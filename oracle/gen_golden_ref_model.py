@@ -41,8 +41,23 @@ def load_reference_model_module():
                 sys.modules[k] = v
 
 
+# Intra-op threads of every run: torch sums train-mode BatchNorm statistics in one partial per thread, so the bits of the
+# train step (which the test demands exactly) depend on the count.  tests/golden/ref_model_standin.pt was made with 8.
+THREADS = 8
+
+
 def run_case(make_net, sizes, k, seed):
-    """One eval forward + one train step under fixed seeds; ``make_net`` builds either implementation."""
+    """One eval forward + one train step under fixed seeds and THREADS threads; ``make_net`` builds either
+    implementation."""
+    threads = torch.get_num_threads()
+    torch.set_num_threads(THREADS)
+    try:
+        return _run_case(make_net, sizes, k, seed)
+    finally:
+        torch.set_num_threads(threads)
+
+
+def _run_case(make_net, sizes, k, seed):
     torch.manual_seed(seed)
     init = O.OracleRandLANet(9, 6, num_neighbors=k, return_logits=True)  # the common initial state
     g = torch.Generator().manual_seed(seed + 1)

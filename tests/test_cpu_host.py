@@ -57,7 +57,9 @@ def test_no_cpu_fallback():
 
 def test_fold_encoder_equals_linear_plus_batchnorm():
     """BN-moment trick (SURVEY.md App. D-7/D-8): folded affine map of q=(p_i,p_j,dist) == Linear(10->h) +
-    train-mode BatchNorm over all edges, values AND gradients AND running statistics (pure torch, CPU)."""
+    train-mode BatchNorm over all edges, values AND gradients AND running statistics (pure torch, CPU).  The unfolded
+    layers run in fp64: the Linear bias gradient is exactly zero under train-mode BatchNorm, and in fp32 torch leaves a
+    residue of up to 4x the tolerance there that depends on how many threads sum the batch statistics."""
     from myria3d_b200.randla_net import SharedMLP, fold_encoder
 
     _, pos, _, ptr = rand_cloud([60, 7], seed=4)
@@ -79,14 +81,15 @@ def test_fold_encoder_equals_linear_plus_batchnorm():
         bn.running_mean.uniform_(-0.3, 0.3, generator=g), bn.running_var.uniform_(0.5, 1.5, generator=g)
         enc = SharedMLP([10, 8])
         enc.load_state_dict(ref.state_dict())
+        ref.double()
         ref.train(training), enc.train(training)
         ref.act = False  # compare pre-activation
-        z_ref = ref(r)
+        z_ref = ref(r.double())
         w, b = fold_encoder(enc, moments, e, training)
         z = q @ w.t() + b
         assert_close(z, z_ref, atol=2e-5, what="folded encoder output")
         go = torch.randn(e, 8, generator=g)
-        z_ref.backward(go)
+        z_ref.backward(go.double())
         z.backward(go)
         for (n1, p1), (_, p2) in zip(enc.named_parameters(), ref.named_parameters()):
             assert_close(p1.grad, p2.grad, atol=2e-4, rtol=2e-4, what=f"fold grad {n1}")
@@ -310,3 +313,28 @@ def test_b200_options_env_is_applied_by_the_binding():
     assert out.stdout.split() == ["3", "1", "31"]
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=ROOT, env=dict(env, B200_OPTIONS="no_such_option=1"))
     assert out.returncode != 0 and "unknown option" in out.stderr
+
+
+def test_bench_dump_outputs_formats_and_size_limit(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 / float64 .npy files, and above the size limit the same fixed, seeded sample of
+    rows of every output with the most rows (row numbers in sample_rows.npy), identical from call to call."""
+    import numpy as np
+
+    import bench
+
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 4096)
+    outs = {"loss": torch.tensor(0.5), "probas": torch.rand(1000, 3), "preds": torch.arange(1000),
+            "stats": torch.rand(7, dtype=torch.float64)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), outs)
+    got = {p.stem: np.load(p) for p in (tmp_path / "a").glob("*.npy")}
+    assert sorted(got) == ["loss", "preds", "probas", "sample_rows", "stats"]
+    assert sum(a.nbytes for a in got.values()) <= 4096
+    assert got["loss"].dtype == np.float32 and got["loss"].tolist() == [0.5]
+    assert got["stats"].dtype == np.float64 and np.array_equal(got["stats"], outs["stats"].numpy())
+    rows = got["sample_rows"].astype(np.int64)
+    assert 0 < len(rows) < 1000 and (np.diff(rows) > 0).all()
+    assert got["probas"].dtype == np.float32 and np.array_equal(got["probas"], outs["probas"].numpy()[rows])
+    assert got["preds"].dtype == np.float64 and np.array_equal(got["preds"], rows)
+    for name, a in got.items():
+        assert np.array_equal(np.load(tmp_path / "b" / f"{name}.npy"), a)

@@ -13,7 +13,7 @@ from oracle.gen_golden import build_net, weight_checksum
 from tests.helpers import assert_close, ptr_of, rand_cloud
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "randla_small.pt")
-CKPT = "/root/reference/trained_model_assets/proto151_V2.0_epoch_100_Myria3DV3.1.0.ckpt"
+CKPT_LAYOUT = os.path.join(os.path.dirname(__file__), "golden", "ref_ckpt_layout.npz")
 
 
 def test_oracle_matches_golden_vectors():
@@ -43,15 +43,21 @@ def test_oracle_matches_golden_vectors():
         assert_close(bufs[k], v, atol=1e-6, rtol=1e-5, what=k)
 
 
-@pytest.mark.skipif(not os.path.exists(CKPT), reason="reference checkpoint not on this box")
-def test_oracle_and_product_strict_load_shipped_checkpoint():
-    """State-dict contract (SURVEY.md App. C): 257 entries, 1 113 719 trainable parameters."""
+def test_oracle_and_product_strict_load_shipped_checkpoint(tmp_path):
+    """State-dict contract (SURVEY.md App. C): 257 entries, 1 113 719 trainable parameters.  The shipped Lightning
+    checkpoint is rebuilt from its pickle and storage layout (tests/golden/ref_ckpt_layout.npz) and its trained weights
+    (tests/golden/randla_trained_ckpt.pt), both taken from the file by oracle/gen_golden_ckpt_layout.py."""
     from myria3d_b200 import B200RandLANet
     from myria3d_b200.ckpt import load_lightning_checkpoint, net_state_dict
+    from oracle.gen_golden_ckpt_layout import rebuild_checkpoint
 
-    ck = load_lightning_checkpoint(CKPT)
+    weights = torch.load(os.path.join(os.path.dirname(__file__), "golden", "randla_trained_ckpt.pt"))["state_dict"]
+    rebuild_checkpoint(CKPT_LAYOUT, weights, str(tmp_path / "shipped.ckpt"))
+    ck = load_lightning_checkpoint(str(tmp_path / "shipped.ckpt"))
+    assert ck["epoch"] == 100 and ck["pytorch-lightning_version"] == "1.5.9"
     sd = net_state_dict(ck)
     assert len(sd) == 257
+    assert sd.keys() == weights.keys() and all(torch.equal(sd[k], v) for k, v in weights.items())
     for cls in (O.OracleRandLANet, B200RandLANet):
         net = cls(9, 7, return_logits=True)
         res = net.load_state_dict(sd, strict=True)
