@@ -34,16 +34,18 @@ int num_sms();
     ::b200::count_launch();                                       \
   } while (0)
 
-// out[m][k] += sum_i a[i][m] * b[i][k]  (a: [n, ca], b: [n, cb], out: [ca, cb]; split-K over n, atomics)
+// out[m][k] += sum_i a[i][m] * b[i][k]  (a: [n, ca], b: [n, cb], out: [ca, cb]; split-K over n).  The attention-weight
+// gradient of the fused LFA backward: n = E edges, up to ~10^6 rows.
 int accumulate_at_b(const float* a, int ca, const float* b, int cb, float* out, int64_t n, float* ws, size_t ws_bytes,
                     cudaStream_t st);
 size_t accumulate_at_b_workspace_bytes(int ca, int cb, int64_t n);
 
 // tensor-core (tcgen05, 3xTF32) version of the same contraction, two-segment activation rows + bias column
 // `ws` (optional, tc_tn_workspace_bytes()): per-split partial tiles + a reduction kernel instead of atomics
+// max_rows_per_split > 0 bounds the rows one CTA accumulates (accuracy of long reductions: tc_gemm.cu)
 int launch_tc_tn(const float* gy, int cout, const float* a1, int64_t ld1, int c1, const float* a2, int64_t ld2, int c2,
-                 float* gw, float* gb, int64_t n, float* ws, size_t ws_bytes, cudaStream_t st);
-size_t tc_tn_workspace_bytes(int cout, int ncols, int64_t n);
+                 float* gw, float* gb, int64_t n, float* ws, size_t ws_bytes, cudaStream_t st, int64_t max_rows_per_split = 0);
+size_t tc_tn_workspace_bytes(int cout, int ncols, int64_t n, int64_t max_rows_per_split = 0);
 // the same contraction for NARROW layers (<= 64 channels, not 64 x 64) on tcgen05 with bf16 x 3 operands read MN-major
 // straight from their row-major layout (tc_skinny.cu)
 bool tc_skinny_tn_ok(int cout, int ktot, bool has_bias, int64_t n);
@@ -56,6 +58,15 @@ int lfa_tc_bwd_dispatch(const float* x, const float* pos, const int32_t* nbr, co
                         const float* att_w, const float* att_wt, const float* go, float* gx, float* gew, float* geb, float* gaw,
                         void* ws, int64_t n, int c, int kt, cudaStream_t st);
 bool lfa_tc_supported(int c, int kt);
+int64_t lfa_tc_bwd_workspace_bytes(int64_t n, int c, int kt);  // when lfa_tc_supported(c, kt)
+// c = 256 (lfa_tc256.cu): W_att streamed from L2 per tile.  The backward writes the fp32 dA and F edge rows
+// (lfa_tc256_bwd_stream_bytes) to ws and reduces dW_att from them with accumulate_at_b, whose partials follow in ws.
+int lfa_tc256_fwd(const float* x, const float* pos, const int32_t* nbr, const float* enc_w, const float* enc_b,
+                  const float* att_wt, float* out, int64_t n, int kt, cudaStream_t st);
+int lfa_tc256_bwd(const float* x, const float* pos, const int32_t* nbr, const float* enc_w, const float* enc_b, const float* att_w,
+                  const float* att_wt, const float* go, float* gx, float* gew, float* geb, float* gaw, const uint32_t* absmax,
+                  float* ws, size_t ws_bytes, int64_t n, int kt, cudaStream_t st);
+size_t lfa_tc256_bwd_stream_bytes(int64_t n, int kt);
 // row-streaming NT GEMM on tcgen05 (tc_nt.cu): out[i][m] = sum_k [a1|a2][i][k] * wm[m][k] + bias[m], channels of the
 // output split over two destination segments; colstats: fp64 (sum, sum of squares) per row tile [tiles][2 * mrows]
 bool tc_nt_shape_ok(int64_t n, int c1, int c2, int mrows);
@@ -90,6 +101,8 @@ bool tc_path_enabled(int bit);  // runtime.cu: b200_set_option("tensor_core_path
 bool tensor_cores_enabled();  // runtime.cu: b200_set_option("tensor_cores", 0) selects the FMA kernels (A/B switch)
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
+// lfa.cu: CTAs of a persistent kernel (resident CTAs per SM x SMs, at most ntiles, at least 1)
+int persistent_grid(const void* kernel, int threads, size_t smem, int64_t ntiles);
 
 constexpr float kLReluSlope = 0.2f;  // pyg_randla_net.py:92
 

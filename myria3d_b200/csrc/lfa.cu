@@ -21,8 +21,9 @@
 //            encoder-gradient partials in shared memory, GEMM3 dW += da^T F as 4x4 register blocks.
 //
 // These FMA kernels serve c in {8, 16} (K = 8 / 16 contractions: 94 % of the edges, too narrow for a 128-lane
-// tensor tile) and c = 256; c in {32, 64, 128} run on tcgen05 (lfa_tc.cu), which maps channels to TMEM lanes and
-// edges to columns so that the same thread-local softmax applies.
+// tensor tile); c in {32, 64, 128, 256} run on tcgen05 (lfa_tc.cu, lfa_tc256.cu), which maps channels to TMEM lanes
+// and edges to columns so that the same thread-local softmax applies.  The FMA kernels of the wider levels stay as
+// the reference of the tensor-core path (b200_set_option("tensor_cores", 0)).
 #include <math_constants.h>
 
 #include "common.cuh"
@@ -735,7 +736,7 @@ static size_t lfa_bwd_smem() {
          sizeof(float) * LfaBwdPlan<Cfg>::GE_SLABS * Cfg::H * 8;
 }
 
-static int persistent_grid(const void* kernel, int threads, size_t smem, int64_t ntiles) {
+int persistent_grid(const void* kernel, int threads, size_t smem, int64_t ntiles) {
   int per_sm = 1;
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem) != cudaSuccess || per_sm < 1) {
     cudaGetLastError();
@@ -820,7 +821,7 @@ extern "C" int b200_lfa_fwd(const float* x, const float* pos, const int32_t* nbr
                "b200_lfa_fwd: x, att_wt and out must be 16-byte aligned");
   if (n <= 0) return B200_OK;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  {  // c in {32, 64, 128}: every contraction on the tensor cores (lfa_tc.cu)
+  {  // c in {32, 64, 128, 256}: the contraction on the tensor cores (lfa_tc.cu, lfa_tc256.cu)
     const int rc = lfa_tc_fwd_dispatch(x, pos, nbr, enc_w, enc_b, att_wt, out, n, c, kt, st);
     if (rc != B200_E_UNSUPPORTED) return rc;
   }
@@ -834,7 +835,7 @@ extern "C" int b200_lfa_fwd(const float* x, const float* pos, const int32_t* nbr
 
 extern "C" int64_t b200_lfa_bwd_workspace_bytes(int64_t n, int32_t c, int32_t kt) {
   if (n <= 0) return 0;
-  if (b200::lfa_tc_supported(c, kt)) return 256;  // tensor-core path: dW_att stays in TMEM; one scratch word (max |grad_out|)
+  if (b200::lfa_tc_supported(c, kt)) return b200::lfa_tc_bwd_workspace_bytes(n, c, kt);
   if (c < 64) return 0;
   return 2 * n * (int64_t)kt * c * (int64_t)sizeof(float) + (int64_t)b200::accumulate_at_b_workspace_bytes(c, c, n * kt);
 }
@@ -856,7 +857,8 @@ extern "C" int b200_lfa_bwd(const float* x, const float* pos, const int32_t* nbr
                B200_E_INVALID, "b200_lfa_bwd: workspace of %lld bytes needed (16-byte aligned)",
                (long long)b200_lfa_bwd_workspace_bytes(n, c, kt));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  {  // c in {32, 64, 128}: every contraction on the tensor cores (lfa_tc.cu)
+  {  // c in {32, 64, 128}: every contraction on the tensor cores (lfa_tc.cu); c = 256 (lfa_tc256.cu): scores and dF
+     // there, dW_att on the split-K tensor-core GEMM
     const int rc = lfa_tc_bwd_dispatch(x, pos, nbr, enc_w, enc_b, att_w, att_wt, grad_out, grad_x, grad_enc_w, grad_enc_b,
                                        grad_att_w, workspace, n, c, kt, st);
     if (rc != B200_E_UNSUPPORTED) return rc;

@@ -2,7 +2,7 @@
 // (tcgen05.mma kind::f16 on fp16 x 2 split operands = fp32-grade products, accumulators in TMEM) -- the
 // c in {32, 64, 128} levels of LocalFeatureAggregation (myria3d/models/modules/pyg_randla_net.py:121-152).
 // Production path of b200_lfa_fwd / b200_lfa_bwd for these widths; narrower levels (c = 8, 16: K = 8 / 16
-// contractions) and c = 256 stay on the FMA kernels of lfa.cu.
+// contractions) stay on the FMA kernels of lfa.cu; c = 256 runs on lfa_tc256.cu (W_att streamed from L2 per tile).
 //
 // Orientation: CHANNELS on the 128 TMEM lanes, the tile's EDGES on the TMEM columns.  An epilogue thread owns one
 // channel and reads, per centre, KT consecutive columns = the neighbours of that centre: the neighbourhood softmax
@@ -50,7 +50,7 @@
 
 #include <type_traits>
 
-#include "tc.cuh"
+#include "lfa_tc.cuh"
 
 namespace b200 {
 
@@ -108,15 +108,9 @@ struct LtcPlan {
   static_assert(SHARED_BYTES % 16 == 0 && SLOT_BYTES % 16 == 0, "alignment");
 };
 
-__device__ __forceinline__ void ltc_wait(uint64_t* bar, uint32_t parity) {
-  if (!tc::mbar_wait_bounded(bar, parity, 20000000u)) __trap();  // a wrong descriptor must not hang the GPU
-}
 __device__ __forceinline__ void slot_sync(int slot) {
   asm volatile("bar.sync %0, %1;" ::"r"(1 + slot), "r"(LTC_SLOT_THREADS) : "memory");
 }
-
-constexpr float kWScale = 16.f;  // W_att is staged as 16 * W (exact): typical weights land in fp16's normal range
-constexpr float kLog2eOverWScale = 1.4426950408889634f / kWScale;
 
 // 4-byte scratch word of the backward: bit pattern of max |grad_out| (non-negative floats order like unsigned ints)
 __global__ void __launch_bounds__(256)
@@ -231,7 +225,7 @@ lfa_tc_kernel(const float* __restrict__ x, const float* __restrict__ pos, const 
   bool mma4_pending = false;
   auto wait_mma4 = [&]() {
     if (mma4_pending) {
-      ltc_wait(bar4, phase4);
+      tc::mbar_wait_or_trap(bar4, phase4);
       tc::fence_after_sync();
       phase4 ^= 1u;
       mma4_pending = false;
@@ -315,60 +309,8 @@ lfa_tc_kernel(const float* __restrict__ x, const float* __restrict__ pos, const 
     if constexpr (BWD) wait_mma4();  // the previous tile's dW MMAs still read F and dA
     slot_sync(slot);
     LTC_TS();
-    // ---- B2 (issue): gathered neighbour features, 8 channels (two 16-byte loads) per item; consumed after B3
-    constexpr int BUILD_ITERS = (NE * H8 + ST - 1) / ST;
-    float4 xa[BUILD_ITERS], xb[BUILD_ITERS];
-#pragma unroll
-    for (int it = 0; it < BUILD_ITERS; ++it) {
-      const int t = it * ST + stid;
-      xa[it] = xb[it] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if ((NE * H8) % ST == 0 || t < NE * H8) {
-        const int j = NB[t / H8];
-        if (j >= 0) {
-          xa[it] = __ldg(reinterpret_cast<const float4*>(x + (int64_t)j * H + 8 * (t % H8)));
-          xb[it] = __ldg(reinterpret_cast<const float4*>(x + (int64_t)j * H + 8 * (t % H8) + 4));
-        }
-      }
-    }
-    // ---- B3: F[:, H:C) = local spatial encoding, 8 channels per item
-#pragma unroll
-    for (int it = 0; it < BUILD_ITERS; ++it) {
-      const int t = it * ST + stid;
-      if ((NE * H8) % ST == 0 || t < NE * H8) {
-        const int e = t / H8, c8 = t % H8;
-        float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-        if (NB[e] >= 0) {
-          const float4 p = P[e / KT], q = Q[e];
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const float4 w0 = EW[17 * c8 + 2 * u], w1 = EW[17 * c8 + 2 * u + 1];
-            float s = fmaf(w0.z, p.z, fmaf(w0.y, p.y, fmaf(w0.x, p.x, w1.w)));
-            s = fmaf(w0.w, q.x, s), s = fmaf(w1.x, q.y, s), s = fmaf(w1.y, q.z, s);
-            s = fmaf(w1.z, q.w, s);
-            v[u] = lrelu(s, kLReluSlope);
-          }
-        }
-        uint4 p1, p2;
-        tc::split8_f16x2(v, p1, p2);
-        const size_t off = ((size_t)(H8 + c8) * (NE + 1) + e) * 16;
-        *reinterpret_cast<uint4*>(Fp + off) = p1;
-        *reinterpret_cast<uint4*>(Fp + Plan::F_PLANE + off) = p2;
-      }
-    }
-    // ---- B2 (consume): F[:, 0:H)
-#pragma unroll
-    for (int it = 0; it < BUILD_ITERS; ++it) {
-      const int t = it * ST + stid;
-      if ((NE * H8) % ST == 0 || t < NE * H8) {
-        const int e = t / H8, m8 = t % H8;
-        const float v[8] = {xa[it].x, xa[it].y, xa[it].z, xa[it].w, xb[it].x, xb[it].y, xb[it].z, xb[it].w};
-        uint4 p1, p2;
-        tc::split8_f16x2(v, p1, p2);
-        const size_t off = ((size_t)m8 * (NE + 1) + e) * 16;
-        *reinterpret_cast<uint4*>(Fp + off) = p1;
-        *reinterpret_cast<uint4*>(Fp + Plan::F_PLANE + off) = p2;
-      }
-    }
+    // ---- B2 / B3: F = [x_j ; lrelu(enc_w . q + enc_b)]
+    ltc_build_f<NE, KT, H, ST>(stid, x, NB, P, Q, EW, Fp, Plan::F_PLANE);
     tc::fence_smem_to_async();
     tc::fence_before_sync();
     slot_sync(slot);
@@ -393,7 +335,7 @@ lfa_tc_kernel(const float* __restrict__ x, const float* __restrict__ pos, const 
       }
       __syncwarp();
     }
-    ltc_wait(bar1, phase);
+    tc::mbar_wait_or_trap(bar1, phase);
     tc::fence_after_sync();
     LTC_TS();
 
@@ -553,7 +495,7 @@ lfa_tc_kernel(const float* __restrict__ x, const float* __restrict__ pos, const 
         __syncwarp();
       }
       mma4_pending = true;
-      ltc_wait(bar3, phase);
+      tc::mbar_wait_or_trap(bar3, phase);
       tc::fence_after_sync();
       LTC_TS();
 
@@ -632,20 +574,8 @@ lfa_tc_kernel(const float* __restrict__ x, const float* __restrict__ pos, const 
       slot_sync(slot);
       tc::fence_after_sync();
       LTC_TS();
-      // ---- scatter the x-gradients: thread = (edge, 4 channels), 16-byte vector reductions
-      constexpr int H4 = H / 4;
-#pragma unroll
-      for (int t0 = 0; t0 < NE * H4; t0 += ST) {
-        const int t = t0 + stid;
-        if ((NE * H4) % ST == 0 || t < NE * H4) {
-          const int e = t / H4, m4 = t % H4;
-          const int j = NB[e];
-          if (j >= 0) {
-            const float4 v = *reinterpret_cast<const float4*>(T + (m4 * (NE + 1) + e) * 4);
-            atomicAdd(reinterpret_cast<float4*>(grad_x + (int64_t)j * H) + m4, v);
-          }
-        }
-      }
+      // ---- scatter the x-gradients
+      ltc_scatter_x<NE, H, ST>(stid, T, NB, grad_x);
       // the next tile's B1 only writes NB / Q / P / DEG, all of which the scatter above still reads
       slot_sync(slot);
       LTC_TS();
@@ -697,10 +627,12 @@ static int launch_lfa_tc(const float* x, const float* pos, const int32_t* nbr, c
 #define B200_LFA_TC_CASES(X) X(32, 16, 128, 128) X(64, 16, 128, 128) X(128, 16, 128, 32) X(64, 32, 128, 128)
 #define B200_LFA_TC_FWD_ONLY_CASES(X) X(128, 32, 64, 0)
 
-// returns B200_E_UNSUPPORTED when this (c, kt) has no tensor-core kernel (the caller then uses the FMA kernel)
+// returns B200_E_UNSUPPORTED when this (c, kt) has no tensor-core kernel (the caller then uses the FMA kernel);
+// c = 256 goes to lfa_tc256.cu
 int lfa_tc_fwd_dispatch(const float* x, const float* pos, const int32_t* nbr, const float* enc_w, const float* enc_b,
                         const float* att_wt, float* out, int64_t n, int c, int kt, cudaStream_t st) {
   if (!tc_path_enabled(16)) return B200_E_UNSUPPORTED;
+  if (c == 256) return lfa_tc256_fwd(x, pos, nbr, enc_w, enc_b, att_wt, out, n, kt, st);
 #define X(C_, KT_, NEF_, NEB_)                                                                                     \
   if (c == C_ && kt == KT_)                                                                                        \
     return launch_lfa_tc<C_, NEF_, KT_, false>(x, pos, nbr, enc_w, enc_b, nullptr, att_wt, out, nullptr, nullptr, nullptr, \
@@ -711,7 +643,14 @@ int lfa_tc_fwd_dispatch(const float* x, const float* pos, const int32_t* nbr, co
   return B200_E_UNSUPPORTED;
 }
 
-// ws: >= 4 bytes of device scratch (the maximum |grad_out| of this call)
+// Backward workspace of the tensor-core path: one scratch word (the maximum |grad_out| of the call), 16-byte aligned;
+// c = 256 adds the fp32 dA and F edge rows and the partials of the split-K dW GEMM behind it.
+int64_t lfa_tc_bwd_workspace_bytes(int64_t n, int c, int kt) {
+  if (c != 256) return 256;  // dW_att stays in TMEM
+  return 16 + (int64_t)lfa_tc256_bwd_stream_bytes(n, kt) + (int64_t)accumulate_at_b_workspace_bytes(c, c, n * kt);
+}
+
+// ws: lfa_tc_bwd_workspace_bytes(n, c, kt) bytes of device scratch
 int lfa_tc_bwd_dispatch(const float* x, const float* pos, const int32_t* nbr, const float* enc_w, const float* enc_b,
                         const float* att_w, const float* att_wt, const float* go, float* gx, float* gew, float* geb, float* gaw, void* ws, int64_t n,
                         int c, int kt, cudaStream_t st) {
@@ -725,6 +664,10 @@ int lfa_tc_bwd_dispatch(const float* x, const float* pos, const int32_t* nbr, co
     lfa_absmax_kernel<<<(unsigned)blocks, 256, 0, st>>>(go, n * c, absmax);
     B200_CHECK_LAUNCH("lfa_absmax_kernel");
   }
+  if (c == 256)
+    return lfa_tc256_bwd(x, pos, nbr, enc_w, enc_b, att_w, att_wt, go, gx, gew, geb, gaw, absmax,
+                         reinterpret_cast<float*>(static_cast<char*>(ws) + 16), (size_t)lfa_tc_bwd_workspace_bytes(n, c, kt) - 16, n,
+                         kt, st);
 #define X(C_, KT_, NEF_, NEB_) \
   if (c == C_ && kt == KT_)    \
     return launch_lfa_tc<C_, NEB_, KT_, true>(x, pos, nbr, enc_w, enc_b, att_w, att_wt, nullptr, go, gx, gew, geb, gaw, absmax, n, st);
@@ -735,6 +678,7 @@ int lfa_tc_bwd_dispatch(const float* x, const float* pos, const int32_t* nbr, co
 
 bool lfa_tc_supported(int c, int kt) {
   if (!tc_path_enabled(16)) return false;
+  if (c == 256 && (kt == 16 || kt == 32)) return true;  // lfa_tc256.cu
 #define X(C_, KT_, NEF_, NEB_) \
   if (c == C_ && kt == KT_) return true;
   B200_LFA_TC_CASES(X)

@@ -15,6 +15,12 @@
 #include "common.cuh"
 
 namespace b200 {
+
+// fused LFA kernels (lfa_tc.cu, lfa_tc256.cu): W_att is staged as 16 * W (exact), so that typical weights land in fp16's
+// normal range; the scores then carry the factor 16
+constexpr float kWScale = 16.f;
+constexpr float kLog2eOverWScale = 1.4426950408889634f / kWScale;
+
 namespace tc {
 
 __device__ __forceinline__ uint32_t lbo_bytes(int rows) { return (uint32_t)(rows + 1) * 16u; }
@@ -208,6 +214,11 @@ __device__ __forceinline__ bool mbar_wait_bounded(uint64_t* bar, uint32_t parity
     if (ok) return true;
   }
   return false;
+}
+
+// the waits of the fused LFA kernels: a wrong descriptor or a lost commit must not hang the GPU
+__device__ __forceinline__ void mbar_wait_or_trap(uint64_t* bar, uint32_t parity) {
+  if (!mbar_wait_bounded(bar, parity, 20000000u)) __trap();
 }
 
 // 16 consecutive fp32 columns of this thread's TMEM lane (warp w of the CTA owns lanes 32*(w%4) .. +31)

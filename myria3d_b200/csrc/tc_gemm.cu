@@ -284,7 +284,9 @@ struct TcTnPlan {
   int64_t splits, rows_per_split;
 };
 
-static TcTnPlan plan_tc_tn(int cout, int ncols, int64_t n) {
+// max_rows_per_split (0: no bound) caps the reduction rows one CTA accumulates in TMEM: the tensor core's fp32 adder
+// truncates, a bias of ~6e-8 of the running sum per MMA, so a split of R rows drifts by ~R / 32 * 12 such steps.
+static TcTnPlan plan_tc_tn(int cout, int ncols, int64_t n, int64_t max_rows_per_split) {
   TcTnPlan p;
   p.bn = (ncols <= 64) ? 64 : ((ncols % 256 == 0) ? 256 : 128);  // 256-wide tiles only when they divide the width
   const int64_t tiles = ceil_div(cout, 128) * ceil_div(ncols, p.bn);
@@ -294,15 +296,17 @@ static TcTnPlan plan_tc_tn(int cout, int ncols, int64_t n) {
   if (splits < 1) splits = 1;
   if (splits > 65535) splits = 65535;
   int64_t rows = ceil_div(n, splits);
+  if (max_rows_per_split > 0 && rows > max_rows_per_split) rows = max_rows_per_split;
+  if (rows < ceil_div(n, 65535)) rows = ceil_div(n, 65535);  // grid.z
   rows = ceil_div(rows, TCG_KC) * TCG_KC;
   p.rows_per_split = rows;
   p.splits = ceil_div(n, rows);
   return p;
 }
 
-size_t tc_tn_workspace_bytes(int cout, int ncols, int64_t n) {
+size_t tc_tn_workspace_bytes(int cout, int ncols, int64_t n, int64_t max_rows_per_split) {
   if (n <= 0) return 0;
-  const TcTnPlan p = plan_tc_tn(cout, ncols, n);
+  const TcTnPlan p = plan_tc_tn(cout, ncols, n, max_rows_per_split);
   return (size_t)p.splits * cout * ((ncols + 3) & ~3) * sizeof(float);
 }
 
@@ -330,10 +334,10 @@ static int launch_tc_tn_bn(const float* gy, int cout, const CatRowsTC& A, float*
 }
 
 int launch_tc_tn(const float* gy, int cout, const float* a1, int64_t ld1, int c1, const float* a2, int64_t ld2, int c2,
-                 float* gw, float* gb, int64_t n, float* ws, size_t ws_bytes, cudaStream_t st) {
+                 float* gw, float* gb, int64_t n, float* ws, size_t ws_bytes, cudaStream_t st, int64_t max_rows_per_split) {
   const CatRowsTC A{a1, ld1, c1, a2, ld2, c2};
   const int ncols = c1 + c2 + (gb ? 1 : 0);
-  const TcTnPlan p = plan_tc_tn(cout, ncols, n);
+  const TcTnPlan p = plan_tc_tn(cout, ncols, n, max_rows_per_split);
   float* partial = (ws && ws_bytes >= (size_t)p.splits * cout * ((ncols + 3) & ~3) * sizeof(float)) ? ws : nullptr;
   if (p.bn == 64) return launch_tc_tn_bn<64>(gy, cout, A, gw, gb, partial, p, n, st);
   if (p.bn == 256) return launch_tc_tn_bn<256>(gy, cout, A, gw, gb, partial, p, n, st);
