@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define B200_ABI_VERSION 5
+#define B200_ABI_VERSION 6
 
 #define B200_OK 0
 #define B200_E_INVALID 1     /* bad argument (null pointer, unsupported size/alignment) */
@@ -365,6 +365,65 @@ int b200_grid_sampling_pool(const uint32_t* key, const uint32_t* val, const int3
 int b200_random_permutation(int64_t n, uint64_t seed, const int64_t* counter, uint32_t salt, uint32_t* key, uint32_t* perm,
                             uint32_t* key_tmp, uint32_t* perm_tmp, const int64_t* offsets01, void* stream);
 int b200_center_pos(float* pos, int32_t n, void* stream);
+
+/* ------------------------------------------------------- batch preparation (train / eval / predict) ------
+ * myria3d's per-sample transform chain, run on a whole raw batch of B samples (sample b = rows [ptr[b], ptr[b+1]) of
+ * pos fp32 [n, 3], x fp32 [n, cx], y int64 [n] raw LAS codes, idx int64 [n] = idx_in_original_cloud), in the order of
+ * pctl/datamodule/hdf5.py:76-89 (preparations + normalizations [+ augmentations in train]).  mode: 0 train, 1 eval,
+ * 2 predict.  Buffers *_c, key / val / *_tmp, run_start and the pooled *_p have the raw layout (n rows, sample b at
+ * ptr[b]); stats is int32 [b200_batch_prep_stats_len(B)]:
+ *   [0] error flags (B200_BATCH_PREP_E_*), [1..8] bitmask of the unknown codes 0..255, [9 + b] rows kept by
+ *   DropPointsByClass, [9 + B + b] voxels after GridSampling.
+ * The caller reads stats once, after _pool, and sizes the rest from it.
+ *
+ * b200_batch_prep_compact replaces TargetTransform (pctl/transforms/transforms.py:168-232: lut[code] = rank in
+ *   classification_dict of preprocessing_dict.get(code, code), 65 for 65, -1 for an unknown code; train / eval only) and
+ *   DropPointsByClass (:235-248: rows labelled 65 dropped, order kept; idx subsampled alike), then computes each sample's
+ *   GridSampling voxel ids over its bounding box (x fastest; B200_BATCH_PREP_E_VOXEL_OVERFLOW when they do not fit
+ *   below 2^32 - 1).  In predict mode lut is ignored and rows with the raw code 65 are dropped.  y / idx may be NULL in
+ *   predict mode.
+ * b200_batch_prep_voxelize: stable per-sample sort of (voxel id, row) and run heads -> run_start, voxel counts.
+ * b200_batch_prep_pool replaces torch_geometric.transforms.GridSampling(grid_size) (points_budget.yaml:76-79): per
+ *   voxel, fp64 mean of pos and x, majority label (ties: lowest class < num_classes); per sample bit-identical to
+ *   b200_grid_sampling_sort / _pool on that sample alone.
+ * b200_batch_prep_budget_draw: the permutations of MinimumNumNodes / MaximumNumNodes (transforms.py:48-84) for the whole
+ *   batch: segment g = [seg_off[g], seg_off[g+1]) (device int64 [num_segments + 1], total = seg_off[num_segments])
+ *   receives a uniformly random permutation of 0 .. length - 1 in perm; seg_ids = int32 [num_segments][2] = (sample,
+ *   repetition) of each segment.  Philox keys of (seed, sample) counted by (row, repetition, *counter) as
+ *   b200_decimation_draw, then b200_segmented_sort_pairs.
+ * b200_batch_prep_finalize: one CTA per sample: rows r < out_ptr[b+1] - out_ptr[b] are pooled rows
+ *   perm[choice_off[b] + r] (choice_off[b] = -1: row r) of sample b; Center (torch_geometric, fp64 mean), NullifyLowestZ,
+ *   NormalizePos (pos * scale, scale = (float)(1 / (subtile_width / 2)), transforms.py:141-165),
+ *   StandardizeRGBAndIntensity on columns col_intensity (log(v + 1) first) and col_rgb (:117-138: fp64 mean and
+ *   unbiased std + 1e-6, NaN std -> 1, clamp to +-3 std), and in train mode RandomFlip(0, flip_p), RandomFlip(1, flip_p)
+ *   (flip_p < 0: none) and RandomRotate(rotate_degrees, axis=2) (0: none; pos @ M^T, M = [[cos, sin, 0], [-sin, cos, 0],
+ *   [0, 0, 1]], cos / sin rounded to fp32) with Philox draws of (seed, *counter, b).  Writes pos_out, x_out, y_out (if
+ *   y_p), batch_out (int64) at out_ptr[b]; eval / predict: pos_sampled_copy (CopySampledPos) and the rows kept by
+ *   DropPointsByClass, pos_c -> pos_copy (CopyFullPos) and, in eval, y_c -> y_copy (CopyFullPreparedTargets) at
+ *   full_ptr[b].  draws (may be NULL) = fp64 [B, 3]: flip x, flip y, angle in degrees. */
+#define B200_BATCH_PREP_E_UNKNOWN_CODE 1
+#define B200_BATCH_PREP_E_CODE_RANGE 2
+#define B200_BATCH_PREP_E_VOXEL_OVERFLOW 4
+int64_t b200_batch_prep_stats_len(int32_t num_samples);
+int b200_batch_prep_compact(int32_t mode, const float* pos, const float* x, int32_t cx, const int64_t* y, const int64_t* idx,
+                            const int64_t* ptr, int32_t num_samples, int64_t n, const int32_t* lut, float grid_size,
+                            float* pos_c, float* x_c, int64_t* y_c, int64_t* idx_c, uint32_t* key, uint32_t* val,
+                            int32_t* stats, void* stream);
+int b200_batch_prep_voxelize(uint32_t* key, uint32_t* val, uint32_t* key_tmp, uint32_t* val_tmp, const int64_t* ptr,
+                             int32_t num_samples, int32_t* run_start, int32_t* stats, void* stream);
+int b200_batch_prep_pool(const uint32_t* val, const int32_t* run_start, const int64_t* ptr, int32_t num_samples, int64_t n,
+                         const int32_t* stats, const float* pos_c, const float* x_c, int32_t cx, const int64_t* y_c,
+                         int32_t num_classes, float* pos_p, float* x_p, int64_t* y_p, void* stream);
+int b200_batch_prep_budget_draw(const int64_t* seg_off, const int32_t* seg_ids, int32_t num_segments, int64_t total,
+                                uint64_t seed, const int64_t* counter, uint32_t* key, uint32_t* perm, uint32_t* key_tmp,
+                                uint32_t* perm_tmp, void* stream);
+int b200_batch_prep_finalize(int32_t mode, const float* pos_p, const float* x_p, int32_t cx, const int64_t* y_p,
+                             const int64_t* ptr, int32_t num_samples, const uint32_t* perm, const int64_t* choice_off,
+                             const int64_t* out_ptr, int32_t col_intensity, int32_t col_rgb, float scale, float flip_p,
+                             float rotate_degrees, uint64_t seed, const int64_t* counter, float* pos_out, float* x_out,
+                             int64_t* y_out, int64_t* batch_out, float* pos_sampled_copy, const float* pos_c,
+                             const int64_t* y_c, const int32_t* stats, const int64_t* full_ptr, float* pos_copy,
+                             int64_t* y_copy, double* draws, void* stream);
 
 /* ------------------------------------------------------- tcgen05 self-test --------------
  * d[128, n] (+)= a[128, k] * b[n, k]^T on the 5th-generation tensor cores (tcgen05.mma, TMEM accumulator):

@@ -36,6 +36,14 @@ _SIGNATURES = {
     "b200_grid_sampling_pool": (c_int, [_P, _P, _P, c_int32, c_int32, _P, _P, c_int32, _P, c_int32, _P, _P, _P, _P, _P]),
     "b200_random_permutation": (c_int, [c_int64, ctypes.c_uint64, _P, ctypes.c_uint32, _P, _P, _P, _P, _P, _P]),
     "b200_center_pos": (c_int, [_P, c_int32, _P]),
+    "b200_batch_prep_stats_len": (c_int64, [c_int32]),
+    "b200_batch_prep_compact": (c_int, [c_int32, _P, _P, c_int32, _P, _P, _P, c_int32, c_int64, _P, c_float, _P, _P, _P, _P, _P,
+                                        _P, _P, _P]),
+    "b200_batch_prep_voxelize": (c_int, [_P, _P, _P, _P, _P, c_int32, _P, _P, _P]),
+    "b200_batch_prep_pool": (c_int, [_P, _P, _P, c_int32, c_int64, _P, _P, _P, c_int32, _P, c_int32, _P, _P, _P, _P]),
+    "b200_batch_prep_budget_draw": (c_int, [_P, _P, c_int32, c_int64, ctypes.c_uint64, _P, _P, _P, _P, _P, _P]),
+    "b200_batch_prep_finalize": (c_int, [c_int32, _P, _P, c_int32, _P, _P, c_int32, _P, _P, _P, c_int32, c_int32, c_float, c_float,
+                                         c_float, ctypes.c_uint64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "b200_tc_gemm_selftest": (c_int, [_P, _P, _P, c_int32, c_int32, c_int32, c_int32, _P, _P]),
     "b200_edge_moments": (c_int, [_P, _P, c_int64, c_int32, _P, _P]),
     "b200_lfa_fwd": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64, c_int32, c_int32, _P]),
@@ -68,7 +76,7 @@ _SIGNATURES = {
     ),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 _lib = None
 

@@ -17,7 +17,7 @@ PKG_DIR = Path(__file__).resolve().parent
 CSRC = PKG_DIR / "csrc"
 BUILD_DIR = PKG_DIR / "csrc" / "build"
 LIB_PATH = PKG_DIR / "libb200randla.so"
-SOURCES = ["runtime.cu", "knn.cu", "knn_grid.cu", "lfa.cu", "lfa_tc.cu", "lfa_tc256.cu", "fold.cu", "pointwise.cu", "linear_rows.cu", "tma_rows.cu", "index_ops.cu", "decimate.cu", "sample_prep.cu", "stitch.cu", "loss.cu", "tc_selftest.cu", "tc_gemm.cu", "tc_nt.cu", "tc_skinny.cu", "optim.cu"]
+SOURCES = ["runtime.cu", "knn.cu", "knn_grid.cu", "lfa.cu", "lfa_tc.cu", "lfa_tc256.cu", "fold.cu", "pointwise.cu", "linear_rows.cu", "tma_rows.cu", "index_ops.cu", "decimate.cu", "sample_prep.cu", "batch_prep.cu", "stitch.cu", "loss.cu", "tc_selftest.cu", "tc_gemm.cu", "tc_nt.cu", "tc_skinny.cu", "optim.cu"]
 ARCH_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a"]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--use_fast_math=false"]
 

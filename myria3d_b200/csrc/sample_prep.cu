@@ -11,6 +11,7 @@
 #include <math_constants.h>
 
 #include "common.cuh"
+#include "sample_prep.cuh"
 
 namespace b200 {
 
@@ -155,15 +156,7 @@ voxel_ids_kernel(const float* __restrict__ pos, int n, float size, const float* 
                  uint32_t* __restrict__ key, uint32_t* __restrict__ val) {
   const int i = blockIdx.x * 256 + threadIdx.x;
   if (i >= n) return;
-  uint32_t id = 0, mul = 1;
-#pragma unroll
-  for (int d = 0; d < 3; ++d) {
-    const float s = start_end[d], e = start_end[3 + d];
-    const uint32_t c = (uint32_t)floorf(__fdiv_rn(__fsub_rn(pos[3 * i + d], s), size));
-    const uint32_t nv = (uint32_t)floorf(__fdiv_rn(__fsub_rn(e, s), size)) + 1u;
-    id += c * mul;
-    mul *= nv;
-  }
+  const uint32_t id = voxel_id(pos + 3 * (int64_t)i, size, start_end);
   key[i] = id;
   val[i] = (uint32_t)i;
 }
@@ -187,51 +180,12 @@ voxel_pool_kernel(const uint32_t* __restrict__ key, const uint32_t* __restrict__
   const int v = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (v >= num_voxels) return;
   const int s = run_start[v], e = (v + 1 < num_voxels) ? run_start[v + 1] : n;
-  const int cols = 3 + cx;
-  for (int c = lane; c < cols; c += 32) {
-    double acc = 0.0;
-    for (int t = s; t < e; ++t) {
-      const int64_t i = val[t];
-      acc += (c < 3) ? (double)pos[3 * i + c] : (double)x[i * cx + (c - 3)];
-    }
-    const float m = (float)(acc / (double)(e - s));
-    if (c < 3)
-      pos_out[3 * (int64_t)v + c] = m;
-    else
-      x_out[(int64_t)v * cx + (c - 3)] = m;
-  }
-  if (y != nullptr) {
-    int best = 0, best_cnt = -1;
-    for (int cl = lane; cl < num_classes; cl += 32) {
-      int cnt = 0;
-      for (int t = s; t < e; ++t) cnt += (y[val[t]] == cl);
-      if (cnt > best_cnt) best_cnt = cnt, best = cl;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      const int oc = __shfl_xor_sync(0xffffffffu, best_cnt, o), ob = __shfl_xor_sync(0xffffffffu, best, o);
-      if (oc > best_cnt || (oc == best_cnt && ob < best)) best_cnt = oc, best = ob;
-    }
-    if (lane == 0) y_out[v] = best;
-  }
+  pool_voxel_run(val, 0, s, e, pos, x, cx, y, num_classes, v, lane, pos_out, x_out, y_out);
   if (lane == 0 && count_out) count_out[v] = e - s;
   (void)key;
 }
 
 // random 32-bit key per element (Philox4x32-10, the stream of decimate.cu) + identity payload
-__device__ __forceinline__ uint32_t sp_philox(uint32_t i_lo, uint32_t i_hi, uint32_t c_lo, uint32_t c_hi, uint32_t k0, uint32_t k1) {
-  uint32_t x0 = i_lo, x1 = i_hi, x2 = c_lo, x3 = c_hi;
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, x0), lo0 = 0xD2511F53u * x0;
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, x2), lo1 = 0xCD9E8D57u * x2;
-    const uint32_t y0 = hi1 ^ x1 ^ k0, y1 = lo1, y2 = hi0 ^ x3 ^ k1, y3 = lo0;
-    x0 = y0, x1 = y1, x2 = y2, x3 = y3;
-    k0 += 0x9E3779B9u;
-    k1 += 0xBB67AE85u;
-  }
-  return x0;
-}
 __global__ void __launch_bounds__(256)
 random_keys_kernel(int64_t n, uint64_t seed, const int64_t* __restrict__ counter, uint32_t salt, uint32_t* __restrict__ key,
                    uint32_t* __restrict__ val) {

@@ -18,7 +18,9 @@ class Data:
         self.__dict__["_store"] = dict(kwargs)
 
     def __getattr__(self, key: str) -> Any:
-        store = self.__dict__["_store"]
+        # .get: while unpickling (DataLoader workers send batches to the main process) the store is not there yet and
+        # pickle probes for __setstate__, which must then be an AttributeError
+        store = self.__dict__.get("_store", {})
         if key in store:
             return store[key]
         raise AttributeError(key)
