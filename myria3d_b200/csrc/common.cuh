@@ -42,10 +42,10 @@ size_t accumulate_at_b_workspace_bytes(int ca, int cb, int64_t n);
 
 // tensor-core (tcgen05, 3xTF32) version of the same contraction, two-segment activation rows + bias column
 // `ws` (optional, tc_tn_workspace_bytes()): per-split partial tiles + a reduction kernel instead of atomics
-// max_rows_per_split > 0 bounds the rows one CTA accumulates (accuracy of long reductions: tc_gemm.cu)
+// (the rows one CTA accumulates are bounded for accuracy of long reductions: tc_gemm.cu)
 int launch_tc_tn(const float* gy, int cout, const float* a1, int64_t ld1, int c1, const float* a2, int64_t ld2, int c2,
-                 float* gw, float* gb, int64_t n, float* ws, size_t ws_bytes, cudaStream_t st, int64_t max_rows_per_split = 0);
-size_t tc_tn_workspace_bytes(int cout, int ncols, int64_t n, int64_t max_rows_per_split = 0);
+                 float* gw, float* gb, int64_t n, float* ws, size_t ws_bytes, cudaStream_t st);
+size_t tc_tn_workspace_bytes(int cout, int ncols, int64_t n);
 // the same contraction for NARROW layers (<= 64 channels, not 64 x 64) on tcgen05 with bf16 x 3 operands read MN-major
 // straight from their row-major layout (tc_skinny.cu)
 bool tc_skinny_tn_ok(int cout, int ktot, bool has_bias, int64_t n);

@@ -499,12 +499,12 @@ static bool tn_uses_tensor_cores(const float* gy, int cout, const CatRows& A, co
 }
 
 static int launch_tn(const float* gy, int cout, const CatRows& A, float* gw, float* gb, int64_t n, float* ws,
-                     size_t ws_bytes, cudaStream_t st, int64_t max_rows_per_split = 0) {
+                     size_t ws_bytes, cudaStream_t st) {
   const int ktot = A.c1 + A.c2;
   const int ncols = ktot + (gb ? 1 : 0);
   // >= 64 x 64 outputs: 5th-generation tensor cores (3xTF32), see tc_gemm.cu
   if (tn_uses_tensor_cores(gy, cout, A, gw, n))
-    return launch_tc_tn(gy, cout, A.a1, A.ld1, A.c1, A.a2, A.ld2, A.c2, gw, gb, n, ws, ws_bytes, st, max_rows_per_split);
+    return launch_tc_tn(gy, cout, A.a1, A.ld1, A.c1, A.a2, A.ld2, A.c2, gw, gb, n, ws, ws_bytes, st);
   {
     // Narrow layers of levels 0-1.  The warp-streaming FMA kernel below reaches 1.3-1.9 TB/s on its vectorised path
     // (cout in {16, 32, 64}, float4-addressable rows); odd shapes (mlp1's 32 -> 4, fc0's 9 -> 32) fall to its scalar
@@ -935,17 +935,13 @@ static int elementwise_grid(int64_t work_items) {
   return (int)(blocks < 1 ? 1 : blocks);
 }
 
-// Over the E edge rows of an LFA level, a split of E / (SMs / tiles) rows accumulated thousands of MMAs into one TMEM
-// accumulator on the larger clouds (the fp32 adder truncates): its dW drifted by up to 5e-5 of scale against fp64.
-// 512 rows per split (192 MMAs) keep it fp32-grade; at the network's level-3 shape that is about the split the plan
-// chose anyway.
-constexpr int64_t kAtBMaxRowsPerSplit = 512;
+// (over the E edge rows of an LFA level the split-K plan bounds the rows one TMEM accumulator sums: tc_gemm.cu)
 int accumulate_at_b(const float* a, int ca, const float* b, int cb, float* out, int64_t n, float* ws, size_t ws_bytes,
                     cudaStream_t st) {
   const CatRows B = make_cat(b, cb, cb, nullptr, 0, 0);
-  return launch_tn(a, ca, B, out, nullptr, n, ws, ws_bytes, st, kAtBMaxRowsPerSplit);
+  return launch_tn(a, ca, B, out, nullptr, n, ws, ws_bytes, st);
 }
-size_t accumulate_at_b_workspace_bytes(int ca, int cb, int64_t n) { return tc_tn_workspace_bytes(ca, cb, n, kAtBMaxRowsPerSplit); }
+size_t accumulate_at_b_workspace_bytes(int ca, int cb, int64_t n) { return tc_tn_workspace_bytes(ca, cb, n); }
 
 }  // namespace b200
 

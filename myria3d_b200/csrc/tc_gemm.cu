@@ -284,9 +284,13 @@ struct TcTnPlan {
   int64_t splits, rows_per_split;
 };
 
-// max_rows_per_split (0: no bound) caps the reduction rows one CTA accumulates in TMEM: the tensor core's fp32 adder
-// truncates, a bias of ~6e-8 of the running sum per MMA, so a split of R rows drifts by ~R / 32 * 12 such steps.
-static TcTnPlan plan_tc_tn(int cout, int ncols, int64_t n, int64_t max_rows_per_split) {
+// A split accumulates its rows in one TMEM accumulator, 12 chained MMAs per 32 rows.  The tensor core's fp32 adder
+// truncates (~6e-8 of the running sum per MMA, always towards zero), so a long split drifts: at myria3d's full
+// 32 x 40 000-point batch the SMs / tiles plan gives 2 000+ rows per split.  Splits longer than kTcTnMaxRowsPerSplit
+// (192 chained MMAs, fp32-grade) are cut into equal parts, so the grid stays a multiple of the one-wave plan.
+constexpr int64_t kTcTnMaxRowsPerSplit = 512;
+
+static TcTnPlan plan_tc_tn(int cout, int ncols, int64_t n) {
   TcTnPlan p;
   p.bn = (ncols <= 64) ? 64 : ((ncols % 256 == 0) ? 256 : 128);  // 256-wide tiles only when they divide the width
   const int64_t tiles = ceil_div(cout, 128) * ceil_div(ncols, p.bn);
@@ -294,9 +298,8 @@ static TcTnPlan plan_tc_tn(int cout, int ncols, int64_t n, int64_t max_rows_per_
   const int64_t max_splits = ceil_div(n, 4 * TCG_KC);
   if (splits > max_splits) splits = max_splits;
   if (splits < 1) splits = 1;
-  if (splits > 65535) splits = 65535;
   int64_t rows = ceil_div(n, splits);
-  if (max_rows_per_split > 0 && rows > max_rows_per_split) rows = max_rows_per_split;
+  if (rows > kTcTnMaxRowsPerSplit) rows = ceil_div(rows, ceil_div(rows, kTcTnMaxRowsPerSplit));
   if (rows < ceil_div(n, 65535)) rows = ceil_div(n, 65535);  // grid.z
   rows = ceil_div(rows, TCG_KC) * TCG_KC;
   p.rows_per_split = rows;
@@ -304,9 +307,9 @@ static TcTnPlan plan_tc_tn(int cout, int ncols, int64_t n, int64_t max_rows_per_
   return p;
 }
 
-size_t tc_tn_workspace_bytes(int cout, int ncols, int64_t n, int64_t max_rows_per_split) {
+size_t tc_tn_workspace_bytes(int cout, int ncols, int64_t n) {
   if (n <= 0) return 0;
-  const TcTnPlan p = plan_tc_tn(cout, ncols, n, max_rows_per_split);
+  const TcTnPlan p = plan_tc_tn(cout, ncols, n);
   return (size_t)p.splits * cout * ((ncols + 3) & ~3) * sizeof(float);
 }
 
@@ -334,10 +337,10 @@ static int launch_tc_tn_bn(const float* gy, int cout, const CatRowsTC& A, float*
 }
 
 int launch_tc_tn(const float* gy, int cout, const float* a1, int64_t ld1, int c1, const float* a2, int64_t ld2, int c2,
-                 float* gw, float* gb, int64_t n, float* ws, size_t ws_bytes, cudaStream_t st, int64_t max_rows_per_split) {
+                 float* gw, float* gb, int64_t n, float* ws, size_t ws_bytes, cudaStream_t st) {
   const CatRowsTC A{a1, ld1, c1, a2, ld2, c2};
   const int ncols = c1 + c2 + (gb ? 1 : 0);
-  const TcTnPlan p = plan_tc_tn(cout, ncols, n, max_rows_per_split);
+  const TcTnPlan p = plan_tc_tn(cout, ncols, n);
   float* partial = (ws && ws_bytes >= (size_t)p.splits * cout * ((ncols + 3) & ~3) * sizeof(float)) ? ws : nullptr;
   if (p.bn == 64) return launch_tc_tn_bn<64>(gy, cout, A, gw, gb, partial, p, n, st);
   if (p.bn == 256) return launch_tc_tn_bn<256>(gy, cout, A, gw, gb, partial, p, n, st);

@@ -8,9 +8,9 @@
 // fp32-grade results.  The bias gradient rides along as one extra column of ones in the activation operand.
 //
 // Persistent CTA per SM: its slab of rows streams through a 2-stage ring (all 256 threads convert chunk t+1 while the
-// tensor core multiplies chunk t: completion through tcgen05.commit -> mbarrier), the [64 x N] accumulator stays in
-// TMEM for the whole slab (M = 64 tile: rows (m % 16) + 32 * (m / 16) of the lane space) and is added to gw / gb with
-// one set of atomics per CTA.  Replaces the warp-streaming FMA kernel tn_skinny_kernel (0.7-1.5 TB/s algorithmic) on
+// tensor core multiplies chunk t: completion through tcgen05.commit -> mbarrier), the [64 x N] accumulator lives in
+// TMEM (M = 64 tile: rows (m % 16) + 32 * (m / 16) of the lane space) for TSK_FLUSH chunks at a time, is then added to
+// fp32 registers, and the slab's sum goes to gw / gb with one set of atomics per CTA.  Replaces the warp-streaming FMA kernel tn_skinny_kernel (0.7-1.5 TB/s algorithmic) on
 // the B200 production path; that kernel stays as the `tensor_cores = 0` fallback.
 #include "tc.cuh"
 
@@ -18,6 +18,10 @@ namespace b200 {
 
 constexpr int TSK_THREADS = 256;
 constexpr int TSK_ROWS = 128;  // rows (K) per chunk
+// The tensor core's fp32 adder truncates (~6e-8 of the accumulator per instruction, always towards zero), so a TMEM
+// chain's bias grows with its length.  A slab is n / 148 rows (8 650 on myria3d's 32 x 40 000-point batch: 68 chunks,
+// 544 chained MMAs): every TSK_FLUSH chunks (64 chained MMAs) the accumulator is added to fp32 registers and restarted.
+constexpr int TSK_FLUSH = 8;
 
 struct TskArgs {
   const float* gy;
@@ -41,9 +45,8 @@ tc_skinny_tn_kernel(const TskArgs p) {
   constexpr size_t G_PLANE = (size_t)MCH * (TSK_ROWS + 1) * 16, A_PLANE = (size_t)NCH * (TSK_ROWS + 1) * 16;
   constexpr size_t STAGE = 3 * (G_PLANE + A_PLANE);
   constexpr int N = NCH * 8;
-  // two accumulators: the t1*t1 products in one, the five small cross products (<= 2^-8 of it) in the other.  The
-  // tensor core's fp32 adder truncates (~6e-8 of the accumulator per instruction, always towards zero), so the bias of
-  // a chain grows with its length: 8 instead of 48 long-chain instructions per chunk keep the slab's sum fp32-grade.
+  // two accumulators: the t1*t1 products in one, the five small cross products (<= 2^-8 of it) in the other: 8 instead
+  // of 48 long-chain instructions per chunk (see TSK_FLUSH for the bound on the chain's length).
   constexpr uint32_t TMEM_COLS = 2 * N <= 32 ? 32 : (2 * N <= 64 ? 64 : 128);
   extern __shared__ __align__(128) unsigned char tsk_smem[];  // 2 stages (+ slack for the M = 64 read of MCH < 8 chunks)
   __shared__ __align__(8) uint64_t bars[2];
@@ -139,6 +142,28 @@ tc_skinny_tn_kernel(const TskArgs p) {
     }
   };
 
+  // TMEM -> registers: warp w reads lane quadrant w % 4 (row m = (lane & 15) + 16 * (w % 4)) and columns
+  // (w / 4) * 16 + 32 * j .. +15 of both accumulators
+  constexpr int NJ = (N + 31) / 32;
+  float racc[NJ][16];
+#pragma unroll
+  for (int j = 0; j < NJ; ++j)
+#pragma unroll
+    for (int u = 0; u < 16; ++u) racc[j][u] = 0.f;
+  auto drain_tmem = [&]() {
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) {
+      const int c0 = (warp >> 2) * 16 + 32 * j;
+      if (c0 < N) {
+        float v[16], w[16];
+        tc::tmem_ld16(tmem_d + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)c0, v);
+        tc::tmem_ld16(tmem_d + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(N + c0), w);
+#pragma unroll
+        for (int u = 0; u < 16; ++u) racc[j][u] += v[u] + w[u];
+      }
+    }
+  };
+
   uint32_t phase[2] = {0, 0};
   int chunk = 0;
   if (row_begin < row_end) load_chunk(row_begin);
@@ -152,6 +177,14 @@ tc_skinny_tn_kernel(const TskArgs p) {
       phase[s] ^= 1u;
     }
     store_chunk(Gp, Ap);
+    if (chunk > 0 && chunk % TSK_FLUSH == 0) {
+      // wait for the previous chunk's MMAs (the phase is not advanced: the wait two chunks on returns at once), add
+      // the accumulator to registers; this chunk's MMAs restart it after the barrier below
+      const int sp = (chunk - 1) & 1;
+      if (!tc::mbar_wait_bounded(&bars[sp], phase[sp], 20000000u)) __trap();
+      tc::fence_after_sync();
+      drain_tmem();
+    }
     tc::fence_smem_to_async();
     tc::fence_before_sync();
     __syncthreads();
@@ -169,7 +202,7 @@ tc_skinny_tn_kernel(const TskArgs p) {
 #pragma unroll
           for (int ks = 0; ks < TSK_ROWS / 16; ++ks)
             tc::mma_bf16(tmem_d + (pass == 0 ? 0u : (uint32_t)N), tc::desc_advance(gd, ks * tc::kPlaneMnStepBytes),
-                         tc::desc_advance(ad, ks * tc::kPlaneMnStepBytes), idesc, chunk != 0 || (pass > 1) || ks != 0);
+                         tc::desc_advance(ad, ks * tc::kPlaneMnStepBytes), idesc, chunk % TSK_FLUSH != 0 || (pass > 1) || ks != 0);
         }
         tc::mma_commit(&bars[s]);
       }
@@ -187,24 +220,22 @@ tc_skinny_tn_kernel(const TskArgs p) {
   }
   tc::fence_after_sync();
   if (chunk > 0) {
+    drain_tmem();
     // M = 64 accumulator: row m sits in TMEM lane (m % 16) + 32 * (m / 16); warps w and w + 4 share a lane quadrant
-    const int lq = warp & 3, lane = tid & 31;
-    const int m = (lane & 15) + 16 * lq;
-    const bool owner = (lane < 16) && (m < p.cout);
-    for (int c0 = (warp >> 2) * 16; c0 < N; c0 += 32) {
-      float v[16], w[16];
-      tc::tmem_ld16(tmem_d + ((uint32_t)(lq * 32) << 16) + (uint32_t)c0, v);
-      tc::tmem_ld16(tmem_d + ((uint32_t)(lq * 32) << 16) + (uint32_t)(N + c0), w);
+    const int lane = tid & 31;
+    const int m = (lane & 15) + 16 * (warp & 3);
+    if ((lane < 16) && (m < p.cout)) {
 #pragma unroll
-      for (int u = 0; u < 16; ++u) v[u] += w[u];
-      if (owner) {
+      for (int j = 0; j < NJ; ++j) {
+        const int c0 = (warp >> 2) * 16 + 32 * j;
+        if (c0 >= N) continue;
 #pragma unroll
         for (int u = 0; u < 16; ++u) {
           const int c = c0 + u;
           if (c < ktot)
-            atomicAdd(p.gw + (int64_t)m * ktot + c, v[u]);
+            atomicAdd(p.gw + (int64_t)m * ktot + c, racc[j][u]);
           else if (c == ktot && p.gb != nullptr)
-            atomicAdd(p.gb + m, v[u]);
+            atomicAdd(p.gb + m, racc[j][u]);
         }
       }
     }
